@@ -16,7 +16,11 @@ buffers per step, > L2 in total, fresh state region per step);
 fpx_step_wait) from pinned host buffers: H2D of the Phase2a and Phase2b batches,
 D2H of the Phase2b and Chosen replies, double-buffered.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+`--dump-outputs DIR` writes what the last timed step returned to its caller as
+DIR/<name>.npy (dump_outputs), so that two builds can be compared output for
+output: every input is generated from fixed seeds.
+
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 """
 import argparse
@@ -65,7 +69,38 @@ def parse():
     ap.add_argument("--cpu-sample-slots", type=int, default=SLOTS_PER_STEP)
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the extra keys (cfg5 on the same GPUs)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the reply streams and watermark of the last timed step as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps the GPU path (--impl ours)")
+    return args
+
+
+DUMP_ROWS = 1 << 20   # rows kept per stream over all ranks: float64 Phase2b + Chosen rows come to 48 MB
+
+
+def dump_outputs(out_dir, rank, n_gpus, r, d_out_p2b, d_out_chosen, d_wm):
+    """What the last timed step returned to its caller: the Phase2b and Chosen streams in emission order, the
+    watermark and the counts fpx_sync reported.  The workload draws no Nack (main asserts n_nack == 0), so the
+    Nack stream is empty and only its count is kept.  float64, because slot numbers outgrow float32's 24-bit
+    mantissa.  A stream longer than DUMP_ROWS / n_gpus rows is stored as a fixed seeded sample of its rows, kept
+    in stream order.  With N > 1 every rank writes its own files (<name>_rank<r>.npy)."""
+    os.makedirs(out_dir, exist_ok=True)
+    cap = DUMP_ROWS // n_gpus
+
+    def rows(t, n):
+        a = t[:n].cpu().numpy().astype(np.float64)
+        if n > cap:
+            a = a[np.sort(np.random.Generator(np.random.PCG64(n)).choice(n, cap, replace=False))]
+        return a
+
+    out = {"phase2b": rows(d_out_p2b, r.n_p2b), "chosen": rows(d_out_chosen, r.n_chosen),
+           "watermark": d_wm.cpu().numpy().astype(np.float64),
+           "sync": np.array([r.status, r.n_p2b, r.n_nack, r.n_chosen, r.watermark], dtype=np.float64)}
+    suffix = "" if n_gpus == 1 else f"_rank{rank}"
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), a)
 
 
 def ncu_traffic(kernel):
@@ -343,6 +378,8 @@ def main():
     assert r.status == 0 and r.n_chosen == SLOTS_PER_STEP and r.n_nack == 0
     exp_wm = (S * SLOTS_PER_STEP) * N + rank
     assert r.watermark == exp_wm, (r.watermark, exp_wm)
+    if args.dump_outputs:    # before the instrumented pass reuses the output buffers
+        dump_outputs(args.dump_outputs, rank, N, r, d_out_p2b, d_out_chosen, d_wm)
     global_prefix = None
     if N > 1:   # every shard's frontier after step S, as the peers stored it into THIS rank's table
         global_prefix, fr = eng.global_watermark(epoch=S)
